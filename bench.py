@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torch.distributed.run, one rank per GPU)
     python bench.py --impl reference ...                     the reference's CPU statement of the path (oracle) on the host cores
+    python bench.py ... --dump-outputs DIR                   also writes the images of the last timed step to DIR/*.npy, to compare builds
 
 Default workload = BVH traversal at the metric's own resolution and bounce count (BASELINE.json configs[2] shape): an
 87,132-triangle mesh in a Cornell room (3 models, BVHs by the reference's builder), 1920x1080, 8 bounces, 256 samples per pixel
@@ -80,6 +81,7 @@ DEFAULT_EXTRA = ["cornell64", "soup4k", "cluster4k", "cornell1", "knot1"]
 EXTRA_STEPS = {"soup4k": (3, 3), "soup4k16": (2, 3), "cluster4k": (4, 3), "cornell1": (64, 8), "knot1": (64, 8)}
 METRIC = "Mrays/s at 1920x1080, 8 bounces (ray = one CalculateRayCollision call)"
 FALLBACK_HBM_GBS = 6650.0
+DUMP_PIXELS = 1 << 20               # --dump-outputs: images above this many pixels are written as this seeded pixel sample (40 MiB in all)
 L2_NOTE = "GPU arm: L2 flushed between steps (256 MiB write inside the timed region); n/a to the CPU arm"
 
 
@@ -317,8 +319,24 @@ def apply_options(ctx, args):
             ctx.set_option(opt, v)
 
 
-def measure(name, w, args, env, steps, warmup, full):
-    """One workload, measured three ways (resident, instrumented replay, end to end).  `full`: also the ncu probe."""
+def dump_outputs(ctx, out_dir):
+    """Writes what the timed path computed in its last step, as a caller of it receives it: the frame image and the accumulated
+    image, (H, W, 4) float32 each.  Larger than DUMP_PIXELS pixels, both are reduced to the same seeded sample of pixels,
+    (DUMP_PIXELS, 4) each, and pixels.npy holds the sampled pixel indices (y * W + x) as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"frame": ctx.readback("FrameRender"), "accumulated": ctx.readback("AccumulatedRender")}
+    h, w = out["frame"].shape[:2]
+    if h * w > DUMP_PIXELS:
+        pix = np.sort(np.random.default_rng(0).choice(h * w, DUMP_PIXELS, replace=False))
+        out = {k: v.reshape(h * w, 4)[pix] for k, v in out.items()}
+        out["pixels"] = pix.astype(np.float64)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
+def measure(name, w, args, env, steps, warmup, full, dump_dir=None):
+    """One workload, measured three ways (resident, instrumented replay, end to end).  `full`: also the ncu probe.
+    `dump_dir`: write the images of the last timed step there (dump_outputs)."""
     torch, dist = env["torch"], env["dist"]
     import ray_tracing_b200 as rt
     from ray_tracing_b200 import build as b, multigpu, scenes
@@ -399,6 +417,8 @@ def measure(name, w, args, env, steps, warmup, full):
     barrier()
     c1 = sampler.mark()
     ms_total = e0.elapsed_time(e1)
+    if dump_dir and rank == 0:
+        dump_outputs(ctx, dump_dir)
     st = ctx.stats()
     rays_local, kernel_ms, exchange_ms = st["rays"], st["kernelMs"], st.get("exchangeMs", 0.0)
 
@@ -592,7 +612,7 @@ def run_gpu(args, name, w):
            "flush": torch.empty(256 << 20, dtype=torch.uint8, device=dev),      # > 126 MB L2
            "l2_peak": measure_l2_peak(torch, dev) if rank == 0 else None}
 
-    main = measure(name, w, args, env, args.steps, args.warmup, full=True)
+    main = measure(name, w, args, env, args.steps, args.warmup, full=True, dump_dir=args.dump_outputs)
     extras = {}
     for xn in args.extra:
         if xn == name:
@@ -647,10 +667,17 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-probe", action="store_true", help="skip the ncu pass (roofline.traffic / physical = null)")
     ap.add_argument("--no-extra-probe", action="store_true", help="ncu pass for the main workload only")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the frame and accumulated images of the main workload's last timed step to DIR/<name>.npy "
+                         "(float32; above 2**20 pixels a seeded sample of 2**20 pixels, their indices in pixels.npy)")
     ap.add_argument("--probe", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--probe-tile", default="0,1,8", help=argparse.SUPPRESS)
     ap.add_argument("--probe-device", type=int, default=0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        raise SystemExit("--dump-outputs: the GPU arm only")
     if args.exchange == "allgather":
         args.exchange = "abi"
     args.extra = [x for x in args.extra.split(",") if x and x != "none"]

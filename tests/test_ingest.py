@@ -55,12 +55,21 @@ def test_obj_loader_without_normals_and_errors(tmp_path):
         rt.load_obj(str(tmp_path / "missing.obj"))
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/Assets/Graphics/Dragon_80K.obj"), reason="reference assets not mounted")
-def test_reference_dragon_loads_and_traces(oracle_path):
-    v, idx, n = rt.load_obj("/root/reference/Assets/Graphics/Dragon_80K.obj")
-    assert idx.size // 3 == 87130                                 # SURVEY.md §0 fact 5
+@pytest.fixture(scope="module")
+def reference_assets(tmp_path_factory):
+    """The original project's Assets: its five scenes and their meshes, cut down (tests/golden/make_reference_excerpt.py)."""
+    from test_round2_abi import extract_reference_excerpt
+    return extract_reference_excerpt(tmp_path_factory.mktemp("reference"))
+
+
+DRAGON_TRIANGLES = 2588             # Dragon_80K.obj (87,130 triangles) decimated; same silhouette
+
+
+def test_reference_dragon_loads_and_traces(oracle_path, reference_assets):
+    v, idx, n = rt.load_obj(os.path.join(reference_assets, "Graphics", "Dragon_80K.obj"))
+    assert idx.size // 3 == DRAGON_TRIANGLES
     tris, nodes, st = rt.build_bvh(v, idx, n)
-    assert st["TriangleCount"] == 87130 and st["LeafDepthMax"] <= 32
+    assert st["TriangleCount"] == DRAGON_TRIANGLES and st["LeafDepthMax"] <= 32
     mesh = scenes.MeshDesc(v, idx, n)
     l2w, w2l = scenes.trs(position=(-0.58, 1.37, 0.09), euler_deg=(0, 59.33, 0), scale=(4.98, 4.98, 4.98))   # Glass Dragon.unity:2075-2088
     sc = scenes.Scene(name="dragon", width=48, height=27, meshes=[mesh],
@@ -114,9 +123,6 @@ def test_display_matches_oracle_on_gpu():
 
 # ---- the reference's serialized scenes (Unity YAML) ---------------------------------------------------------------------------
 
-SCENES_DIR = "/root/reference/Assets/Scenes"
-
-
 def test_exr_export_is_lossless(tmp_path, oracle_path):
     """The float4 accumulation buffer through write_exr / read_exr: bit-identical, NaN and inf included; header fields as the format wants."""
     _, accum = render(oracle_path, scenes.cornell_spheres(37, 21, 3, 2), frames=2)
@@ -144,9 +150,9 @@ def test_builtin_unity_meshes():
     assert quad.triangle_count == 2 and np.allclose(quad.normals, [[0, 0, -1]] * 4)
 
 
-@pytest.mark.skipif(not os.path.isdir(SCENES_DIR), reason="reference scenes not mounted")
-def test_reference_scenes_load_with_the_serialized_settings(oracle_path):
+def test_reference_scenes_load_with_the_serialized_settings(oracle_path, reference_assets):
     from ray_tracing_b200 import unity_scene
+    SCENES_DIR = os.path.join(reference_assets, "Scenes")
     expect = {   # SURVEY.md Appendix B
         "Glass Dragon": dict(models=11, bounces=10, fov=54.5, cam=(0.0, 1.9, -5.67), diverge=1.5, defocus=0.0),
         "Glass Balls": dict(models=17, bounces=10, fov=60.0, cam=(0.0, 1.99, -5.895), diverge=1.5, defocus=0.0),
@@ -160,7 +166,7 @@ def test_reference_scenes_load_with_the_serialized_settings(oracle_path):
     assert sc.settings["focusDistance"] == pytest.approx(5.3)      # Sphere Refract: depth of field
     # Glass Dragon: the dragon mesh is the shipped OBJ, glass, as serialized (Glass Dragon.unity:1988-2073)
     sc = unity_scene.load_unity_scene(os.path.join(SCENES_DIR, "Glass Dragon.unity"), width=64, height=36)
-    dragon = [m for m in sc.models if sc.meshes[m.mesh].triangle_count == 87130]
+    dragon = [m for m in sc.models if sc.meshes[m.mesh].triangle_count == DRAGON_TRIANGLES]
     assert len(dragon) == 1 and int(dragon[0].material["flag"]) == scenes.MAT_GLASS and float(dragon[0].material["ior"]) == 1.5
     assert np.allclose(np.linalg.norm(dragon[0].local_to_world[:3, 0]), 4.98, atol=1e-2)
     sc.settings["numRaysPerPixel"] = 16
@@ -265,14 +271,15 @@ def test_unity_mesh_file_ids_known_answers():
         assert fbx_mesh.unity_mesh_file_id(name) == fid, name
 
 
-@pytest.mark.skipif(not os.path.isdir(SCENES_DIR), reason="reference scenes not mounted")
-def test_reference_fbx_scenes_load_and_trace(oracle_path):
-    """Text.unity (ten glyph meshes of Text.fbx, normals recomputed as its .meta asks) and Splash.unity (Water.fbx, 656,796
-    triangles, bvhQuality Low): every mesh id resolves, the geometry sits inside the room, the scene traces."""
+def test_reference_fbx_scenes_load_and_trace(oracle_path, reference_assets):
+    """Text.unity (ten glyph meshes of Text.fbx, normals recomputed as its .meta asks) and Splash.unity (Water.fbx, bvhQuality Low),
+    with every geometry of both files cut to its first polygons plus the ones that hold its extreme vertices: every mesh id resolves,
+    the geometry sits inside the room, the scene traces."""
     from ray_tracing_b200 import unity_scene
+    SCENES_DIR = os.path.join(reference_assets, "Scenes")
     sc = unity_scene.load_unity_scene(os.path.join(SCENES_DIR, "Text.unity"), width=64, height=36)
-    glyphs = sorted(m.triangle_count for m in sc.meshes if m.triangle_count not in (2, 12, 87130))
-    assert glyphs == [284, 284, 2444, 2736, 3740, 4364, 4364, 6048, 6048, 6956] and len(sc.models) == 18      # the ten glyph meshes of Text.fbx
+    glyphs = sorted(m.triangle_count for m in sc.meshes if m.triangle_count not in (2, 12, DRAGON_TRIANGLES))
+    assert glyphs == [100, 101, 107, 114, 116, 120, 121, 123, 124, 126] and len(sc.models) == 18      # the ten glyph meshes of Text.fbx
     for md in sc.models:
         m = sc.meshes[md.mesh]
         w = (md.local_to_world[:3, :3] @ m.vertices.T.astype(np.float64)).T + md.local_to_world[:3, 3]
@@ -281,7 +288,7 @@ def test_reference_fbx_scenes_load_and_trace(oracle_path):
     frame, _ = render(oracle_path, sc)
     assert np.isfinite(frame).all() and (frame[..., :3].sum(-1) > 0).mean() > 0.05     # one small ceiling light: a dark, noisy room
     sp = unity_scene.load_unity_scene(os.path.join(SCENES_DIR, "Splash.unity"), width=48, height=27)
-    water = [m for m in sp.models if sp.meshes[m.mesh].triangle_count == 656796]
+    water = [m for m in sp.models if sp.meshes[m.mesh].triangle_count == 1505]
     assert len(water) == 1 and sp.settings["bvhQuality"] == 0
     m = sp.meshes[water[0].mesh]
     w = (water[0].local_to_world[:3, :3] @ m.vertices.T.astype(np.float64)).T + water[0].local_to_world[:3, 3]

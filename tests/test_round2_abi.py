@@ -274,7 +274,16 @@ def test_cpp_tiled_example_on_the_interpreter_build(tmp_path, simt_lib, oracle_p
 # ---- an ingested scene (SURVEY 8f #2): the committed Unity-YAML + OBJ fixture -----------------------------------------------------
 
 FIXTURE_SCENE = os.path.join(REPO, "tests", "fixtures", "unity_project", "Assets", "Scenes", "Fixture.unity")
-REFERENCE_SCENES = "/root/reference/Assets/Scenes"
+REFERENCE_EXCERPT = os.path.join(REPO, "tests", "golden", "reference_excerpt.tar.xz")
+
+
+def extract_reference_excerpt(dest) -> str:
+    """Unpacks the original project's five scenes with their meshes cut down (tests/golden/make_reference_excerpt.py) into `dest`;
+    returns the Assets directory."""
+    import tarfile
+    with tarfile.open(REFERENCE_EXCERPT) as tar:
+        tar.extractall(str(dest), filter="data")
+    return os.path.join(str(dest), "Assets")
 
 
 def load_fixture(width=None, height=None):
